@@ -16,7 +16,20 @@ Three legs, all on THE SAME 1024 synthetic rays per GPU (nero_b200.synthetic.syn
           `e2e.train_ray_num_512`;
   bear    the same resident loop on BASELINE.json configs[2] (human light, 2048 rays on one GPU; 1024 per GPU under
           torchrun = configs[4] at 8 GPUs), reported under the key "bear" of the same JSON line.
-Prints ONE JSON line (see the driver contract in the task statement).
+--steps sets the number of timed steps of every leg above and of the reference arm.  Fixed-size samples that --steps does
+not set: the cpu_baseline records (2 timed steps each on the host CPU: 256 rays of this workload, and BASELINE.json
+configs[0] at steps 10000 and 30000), and the one extra step the chain roofline is profiled on.  Prints ONE JSON line on
+stdout.
+
+    python bench.py --dump-outputs DIR ...                         # also write resident-step outputs to DIR
+
+--dump-outputs writes, after the resident leg's timed steps, what its last step computed as DIR/<name>.npy (float32, rank
+0's shard): z_vals, the render_core outputs, the loss, and the gradients and updated parameters (flattened in parameter
+order).  The same arrays of the first warm-up step, which starts from the seeded initial parameters, go to
+DIR/first_step_<name>.npy.  The inputs are seeded, so two builds run with the same arguments can be compared output for
+output.  Parameter gradients are summed with fp32 atomics, and every step before the last one feeds them to Adam, so two
+runs of one build differ in the last step's parameters and outputs by that rounding compounded over warmup + steps
+updates; the first step carries only one step's rounding and is the tighter comparison.
 """
 import argparse
 import json
@@ -39,6 +52,7 @@ A_SDF, A_SHADE, A_SHADE_H, A_NERF = 524544, 1211648, 1349888, 604160   # MAC / s
 STEP = 30000
 RAYS_PER_GPU = 1024
 METRIC = 'train rays/sec (128 samples/ray)'
+DUMP_BYTES = 64 << 20       # --dump-outputs budget (about 38 MB are written at the default workload)
 
 
 def workload_config(bear, R, world):
@@ -171,7 +185,7 @@ class Workload:
         n = e.state['N_in'] if e.state['N_in'] is not None else e.w['n_in']      # graph mode keeps the count on the device
         return self.dp.global_mean_weight(n, self.world)
 
-    def resident_step(self):
+    def resident_step(self, keep=False):
         net, r, R = self.net, self.r, self.R
         self.opt.zero_grad(set_to_none=True)
         ri = torch.rand([R, 1], device=self.dev, generator=self.gen)
@@ -182,6 +196,8 @@ class Workload:
         loss.backward()
         self.sync_grads()
         self.opt.step()
+        if keep:        # for step_arrays (--dump-outputs)
+            self.last = {'z_vals': z, **out, 'loss': loss}
         return loss
 
     def e2e_step(self, step):
@@ -196,6 +212,24 @@ class Workload:
     def counts(self):
         st = self.net.engine.state
         return st['N_in'], int(self.net.engine.w['n_out'].item()), st['P']
+
+
+def step_arrays(wl):
+    """Host float32 copies of what `wl.resident_step(keep=True)` computed: its outputs, gradients and updated parameters."""
+    arrays = {k: v.detach() for k, v in wl.last.items()}
+    arrays['grads'] = torch.cat([p.grad.reshape(-1) for p in wl.params])
+    arrays['params'] = torch.cat([p.detach().reshape(-1) for p in wl.params])
+    return {k: v.float().cpu().numpy() for k, v in arrays.items()}
+
+
+def dump_outputs(out_dir, last, first):
+    """Writes step_arrays of the last timed step as <name>.npy and of the first warm-up step as first_step_<name>.npy."""
+    arrays = {**last, **{'first_step_' + k: v for k, v in first.items()}}
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= DUMP_BYTES, f'--dump-outputs: {total} bytes exceed the {DUMP_BYTES}-byte budget'
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + '.npy'), a)
 
 
 def timed(fn, steps, barrier):
@@ -245,16 +279,21 @@ def run_ours(args):
     bear = args.workload == 'bear'
     wl = Workload(bear, rank, world, dev)
     R = wl.R
-    for _ in range(args.warmup):
-        wl.resident_step()
+    dump = bool(args.dump_outputs) and rank == 0
+    for i in range(args.warmup):
+        wl.resident_step(keep=dump and i == 0)
+        if dump and i == 0:
+            first = step_arrays(wl)
     barrier()
     sampler = ClockSampler(local)      # clocks / throttle reasons of rank 0's GPU only (one nvidia-smi poller per job, not per rank)
     if rank == 0:
         sampler.start()
     l0 = ops.launch_count
-    ms = timed(lambda i: wl.resident_step(), args.steps, barrier)
+    ms = timed(lambda i: wl.resident_step(keep=dump and i == args.steps - 1), args.steps, barrier)
     launches = (ops.launch_count - l0) // args.steps
     n_in, n_out, p_occ = wl.counts()
+    if dump:
+        dump_outputs(args.dump_outputs, step_arrays(wl), first)
 
     # ---- end to end through the public API with host buffers (H2D of the ray batch + D2H of the loss every step):
     # the headline leg replays the step from CUDA graphs (cfg['cuda_graph']); the eager leg and the reference's default
@@ -289,11 +328,10 @@ def run_ours(args):
         wb = Workload(True, rank, world, dev)
         for _ in range(3):
             wb.resident_step()
-        ksteps = max(3, min(args.steps, 10))
-        ms_b = timed(lambda i: wb.resident_step(), ksteps, barrier)
+        ms_b = timed(lambda i: wb.resident_step(), args.steps, barrier)
         nb_in, nb_out, pb = wb.counts()
         ms_b, = reduce_max([ms_b])
-        other = {'metric': METRIC, 'value': wb.R * world / (ms_b * 1e-3), 'unit': 'rays/s', 'ms_per_step': ms_b, 'steps': ksteps, 'warmup': 3,
+        other = {'metric': METRIC, 'value': wb.R * world / (ms_b * 1e-3), 'unit': 'rays/s', 'ms_per_step': ms_b, 'steps': args.steps, 'warmup': 3,
                  'config': workload_config(True, wb.R, world), 'counts': {'n_in': nb_in, 'n_out': nb_out, 'p_occ': pb},
                  'step_tensor_tflops': algorithmic_flops(wb.R, nb_in, nb_out, pb, True) / (ms_b * 1e-3) / 1e12}
         del wb
@@ -455,8 +493,8 @@ def cpu_baseline_default():
 
 def run_reference(args):
     """The reference arm: the reference's algorithm (bit-exact CPU port) on all host cores, on the headline configuration
-    itself -- every step is the full 1024-ray x (64+64)+32 batch of configs[1] (about 10 s per step on 8 cores), so the number
-    of timed steps is bounded by a time budget rather than by --steps."""
+    itself -- every step is the full 1024-ray x (64+64)+32 batch of configs[1] (about 10 s per step on 8 cores); --steps
+    sets the number of timed steps (--steps 2 for a short run)."""
     rank = int(os.environ.get('RANK', 0))
     world = int(os.environ.get('WORLD_SIZE', 1))
     if rank != 0:
@@ -465,7 +503,7 @@ def run_reference(args):
     R = rays_per_gpu(bear, world)
     cfg = {'shader_config': {'human_light': True}} if bear else {}
     t0 = time.time()
-    steps = max(1, min(args.steps, 2))
+    steps = args.steps
     cb = cpu_baseline(rays_n=R, steps=steps, cfg=cfg)
     c0 = {'n_samples': 32, 'n_importance': 32}
     extra = {f'step{s}': {k: v for k, v in cpu_baseline(256, 2, cb['cores'], c0, s).items() if k in ('value', 'seconds_per_step', 'sample')}
@@ -476,7 +514,7 @@ def run_reference(args):
             'config': workload_config(bear, R, world),
             'note': 'the reference is a pure-PyTorch script repository that cannot be installed or shipped to the GPU box; this is its '
                     'bit-exact CPU port (oracle/nero_oracle.py, pinned by tests/golden) on the host cores, one rank, timing the '
-                    f'full per-GPU batch of the workload ({R} rays) per step; steps bounded to {steps} (about 10 s each)',
+                    f'full per-GPU batch of the workload ({R} rays) per step; {steps} timed steps (about 10 s each)',
             'config0_256rays_x_(32+32)+32': extra, 'wall_s': time.time() - t0,
             'cpu_baseline': cb,
             'e2e': {'value': cb['value'], 'unit': 'rays/s', 'h2d_bytes_per_step': 0, 'd2h_bytes_per_step': 0}}
@@ -493,7 +531,12 @@ def main():
                     help="bell = BASELINE.json configs[1] (the headline, default); bear = configs[2]: human light, 2048 rays")
     ap.add_argument('--no-cpu', action='store_true', help='skip the cpu_baseline leg (profiling runs)')
     ap.add_argument('--no-bear', action='store_true', help='skip the second workload (configs[2]) record')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write the outputs of the last timed resident step to DIR/<name>.npy and of the first warm-up step to '
+                         'DIR/first_step_<name>.npy (float32)')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
     args.warmup = max(args.warmup, 3)
     if args.impl == 'reference':
         run_reference(args)

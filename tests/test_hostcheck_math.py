@@ -172,7 +172,7 @@ def test_sphere_direction(hc):
 def test_combine(hc):
     g = torch.Generator().manual_seed(7)
     n = 600
-    lut = torch.from_numpy(np.fromfile('assets/bsdf_256_256.bin', dtype=np.float32).reshape(256, 256, 2).copy())
+    lut = torch.from_numpy(np.fromfile(os.path.join(HERE, '..', 'assets', 'bsdf_256_256.bin'), dtype=np.float32).reshape(256, 256, 2).copy())
     x = torch.rand(n, 20, generator=g)
     x[:, 14] = torch.randn(n, generator=g) * 1.5          # inner weight (occ clamp both sides)
     x[:, 19] = torch.rand(n, generator=g) * 1.4 - 0.2     # NoV beyond [0,1]

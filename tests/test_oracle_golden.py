@@ -1,5 +1,7 @@
 """Pins oracle/nero_oracle.py to the golden vectors produced by the UNMODIFIED reference
 (oracle/make_golden.py).  CPU only."""
+import os
+
 import numpy as np
 import pytest
 import torch
@@ -8,6 +10,8 @@ import nero_oracle as O
 import nero_oracle_mat as OM
 from helpers import load_golden, build_params, param_checksums, t, rays_from_golden, FIXTURE_CFGS, FIXTURE_STEPS, VAL_FIXTURES
 from helpers import MATERIAL_FIXTURES, build_material_params, material_batch_from_golden, material_rands
+
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 def test_encoding_kats():
@@ -30,7 +34,7 @@ def test_known_answers_from_survey():
     d = torch.nn.functional.normalize(torch.tensor([[1e-6, 1e-6, 1.0]]), dim=-1)
     e = O.ide(d, torch.zeros(1, 1))[0]
     np.testing.assert_allclose(e[[0, 2, 5, 10, 19]].numpy(), [0.4886, 0.6308, 0.8463, 1.1631, 1.6221], atol=2e-4)
-    lut = torch.from_numpy(np.fromfile('assets/bsdf_256_256.bin', dtype=np.float32).reshape(256, 256, 2).copy())
+    lut = torch.from_numpy(np.fromfile(os.path.join(ROOT, 'assets', 'bsdf_256_256.bin'), dtype=np.float32).reshape(256, 256, 2).copy())
     # LUT corner KATs: uv = [NoV, roughness] -> lut[row=roughness, col=NoV]
     for uv, want in [((0.0, 0.0), (0.00972746, 0.9902487)), ((1.0, 0.0), (1.0, 2.84e-14)),
                      ((0.0, 1.0), (0.941525, 0.04653827)), ((1.0, 1.0), (0.30927664, 3.5468642e-05))]:
